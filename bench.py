@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the create_proof hot path (BASELINE.json configs[1]):
 BN254 G1 Pippenger MSM over 2^20 random points / uniform scalars per GPU, B200 vs the CPU best_multiexp.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one batch of MSMS_PER_STEP = 16 commitments, each an MSM of n = 2^20 pairs per GPU against a resident basis
@@ -38,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is written there, bytecode caches included
 
 LOG_N = 20
 N_PAIRS = 1 << LOG_N
@@ -119,6 +120,17 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": float(np.median(self.samples)) if self.samples else None, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
 
 
+def dump_commitments(out_dir, name, jacobian):
+    """(count, 12) Jacobian Montgomery limbs -> out_dir/<name>.npy, float64 of shape (count, 2, 8): the affine x and y of each
+    point as eight little-endian 32-bit limbs, which float64 holds exactly (the identity is x = y = 0). Affine coordinates
+    are unique, so two builds that compute the same points write the same file."""
+    from spectre_b200 import halo2
+    xy = [halo2.jacobian_to_affine_ints(j) for j in np.asarray(jacobian, dtype=np.uint64).reshape(-1, 12)]
+    limbs = np.array([[[(v >> (32 * i)) & 0xFFFFFFFF for i in range(8)] for v in p] for p in xy], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), limbs)
+
+
 def dist_env():
     return int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 
@@ -164,8 +176,10 @@ def run_reference(args):
     ts = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        orc.best_multiexp(sc, bases, threads=threads)
+        res = orc.best_multiexp(sc, bases, threads=threads)
         ts.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_commitments(args.dump_outputs, "msm_commitments", res)
     med = float(np.median(ts))
     val = N_PAIRS / med
     line = {
@@ -212,14 +226,11 @@ def main():
     ap.add_argument("--prove-k", type=int, default=23, help="k of the aggregation-shaped proof")
     ap.add_argument("--prove-k-step", type=int, default=20, help="k of the sync-step-shaped proof")
     ap.add_argument("--no-tables", action="store_true", help="skip spb_srs_precompute (W separate bucket sets, Horner over windows)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the commitments of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
-        if args.steps > 7:
-            args.steps = 7   # each step is a full 2^20 MSM on the CPU (0.3 - 1.5 s on the pool's hosts)
-        if args.steps < 5:
-            args.steps = 5
         return run_reference(args)
 
     import torch
@@ -318,6 +329,9 @@ def main():
     stages_pipelined = be.last_msm_stage_ms         # last MSM of the timed batch (other lane running concurrently)
     e2e_steps = max(3, args.steps // 2)
     e2e_wall_ms = timed(run_e2e, e2e_steps, 3)
+    if args.dump_outputs and rank == 0:
+        dump_commitments(args.dump_outputs, "msm_commitments", last["dev"][1])
+        dump_commitments(args.dump_outputs, "msm_commitments_e2e", last["e2e"][1])
 
     # ---- parity of the timed path: last timed step, first MSM of the batch, vs (sum s_i h_i) * G1 from the oracle ------
     parity = {}
@@ -718,6 +732,7 @@ def prove_both(torch, halo2, be, args):
     from tools import cpp_driver
     secret = plonk.fr_mont(0x5eed7a75)                        # any SRS secret: timings do not depend on it
     proofs = {}
+    exe, exe_dir = None, tempfile.TemporaryDirectory()        # the compiled driver is built outside the tree, which may be read-only
     for name, k in (("sync_step_shape", args.prove_k_step), ("aggregation_shape", args.prove_k)):
         t0 = time.perf_counter()
         srs = halo2.ParamsKZG.setup(be, k, secret).precompute()
@@ -747,8 +762,8 @@ def prove_both(torch, halo2, be, args):
                 E.sync(); t_py_host_rng = time.perf_counter() - t0
                 del E, pkey, srs
                 torch.cuda.empty_cache()
-                exe = cpp_driver.build_main_against_the_real_library()
-                with tempfile.TemporaryDirectory(dir="/tmp") as d:
+                exe = exe or cpp_driver.build_main_against_the_real_library(out_dir=exe_dir.name)
+                with tempfile.TemporaryDirectory() as d:
                     head = "shape aggregation" if name == "aggregation_shape" else "shape halo2lib 15 2"
                     cpp_driver.dump_case(d, head, k, BENCH_VK_DIGEST, inst, copies, rec.counts, fixed_cols, adv_cols, rec.rows, secret, chacha_poly=host.chacha_seed)
                     rc, log, cproof, ms, kg = cpp_driver.run(exe, d, repeat=3, tables=True)
@@ -765,6 +780,7 @@ def prove_both(torch, halo2, be, args):
         E = pkey = srs = None
         del fixed_cols, adv_cols, pinned
         torch.cuda.empty_cache()
+    exe_dir.cleanup()
     proofs["sync_step_compressed_shape_total_s"] = proofs["sync_step_shape"]["create_proof_s"] + proofs["aggregation_shape"]["create_proof_s"]
     proofs["what"] = ("create_proof wall seconds, best warm pass of 2: pinned witness H2D, blinding, every commitment, evaluate_h, evaluations, SHPLONK, Keccak transcript; "
                       "host driver in Python over the C ABI (no torch synchronisation: everything is ordered on the library's stream); synthetic witnesses with full "

@@ -88,67 +88,67 @@ def _fixtures():
     return sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "aggregation_k*_proof.json")))
 
 
-@pytest.mark.skipif(not __import__("tests.yul_harness", fromlist=["x"]).available(), reason="reference tree not present")
-@pytest.mark.parametrize("path", _fixtures(), ids=lambda p: p.split("_")[-2])
-def test_reference_verifier_contract_accepts_the_fixture(orc, kats, path):
-    """contracts/snark-verifiers/{sync_step,committee_update}_verifier.sol, interpreted as they stand in the reference tree,
-    accept the committed proofs (VK commitments substituted, pairing decided with the known tau: tests/yul_harness.py), and
-    reject them after a one-bit change or with a different public input."""
+def _contract_run(path):
+    """the fixture's inputs and what the reference's verifier contract did with them: tests/golden/verifier_contract_runs.json,
+    recorded by tools/extract_golden.py with tests/yul_harness.py (VK commitments substituted, pairing decided with the known tau)"""
     import json
     import os
     from tests import yul_harness
     with open(path) as f:
         fx = json.load(f)
-    contract = fx.get("contract", "sync_step_verifier")
-    instances = [int(v, 16) for v in fx["instances"]]
-    proof = bytes.fromhex(fx["proof"])
-    vk_points = [(int(x, 16), int(y, 16)) for x, y in fx["vk_points"]]
-    tau = orc.fr_ints(orc.srs_tau().reshape(1, 4))[0]
-    ok, m = yul_harness.run_contract(contract, instances, proof, vk_points, tau, kats)
-    assert ok and m.pairing_calls == 1 and m.precompile_counts[7] == 21
-    bad = bytearray(proof); bad[11 * 64 - 1 + 32 * 3] ^= 1         # one bit of an evaluation
-    assert not yul_harness.run_contract(contract, instances, bytes(bad), vk_points, tau, kats)[0]
-    assert not yul_harness.run_contract(contract, instances[:-1] + [instances[-1] + 1], proof, vk_points, tau, kats)[0]
-    # control: with the contract's own VK constants (the real circuit's fixed columns, not ours) the same proof must fail,
-    # and so must a wrong tau in the pairing decision
-    with open(os.path.join(yul_harness.REF_DIR, contract + ".sol")) as f:
-        own = yul_harness.vk_literals(f.read())
-    assert own[1] == vk_points[1] and own[0] != vk_points[0]      # only the range table coincides
-    assert not yul_harness.run_contract(contract, instances, proof, own, tau, kats)[0]
-    assert not yul_harness.run_contract(contract, instances, proof, vk_points, tau + 1, kats)[0]
-    # and the independent Python verifier agrees on the same bytes
-    from tests import plonk_verifier
-    cs = plonk_circuits.aggregation_shape()
-    assert plonk_verifier.verify(cs, fx["k"], int(fx["vk_digest"]), vk_points[:4], vk_points[4:], [instances], proof, tau)
+    with open(os.path.join(os.path.dirname(__file__), "golden", "verifier_contract_runs.json")) as f:
+        run = json.load(f)[os.path.basename(path)]
+    contract, instances, proof, vk_points = yul_harness.fixture_inputs(fx)
+    assert run["contract"] == contract and run["inputs_keccak"] == yul_harness.inputs_digest(instances, proof, vk_points), \
+        "the recorded contract run is not of this fixture: re-run tools/extract_golden.py"
+    return fx, run, instances, proof, vk_points
 
 
 @pytest.mark.parametrize("path", _fixtures(), ids=lambda p: p.split("_")[-2])
-def test_independent_verifier_agrees_with_the_contract_term_by_term(orc, kats, path):
+def test_reference_verifier_contract_accepts_the_fixture(orc, path):
+    """contracts/snark-verifiers/{sync_step,committee_update}_verifier.sol, interpreted as they stand in the reference tree,
+    accepted the committed proofs and rejected them after a one-bit change, with a different public input, with the
+    contract's own VK constants and with a wrong tau; the independent Python verifier reaches the same verdict on each."""
+    from tests import plonk_verifier, yul_harness
+    fx, run, instances, proof, vk_points = _contract_run(path)
+    tau = orc.fr_ints(orc.srs_tau().reshape(1, 4))[0]
+    assert run["verdicts"] == {"fixture": True, "flipped_evaluation_bit": False, "changed_public_input": False, "contract_vk_constants": False,
+                               "wrong_tau": False}
+    assert run["pairing_calls"] == 1 and run["precompile_counts"]["7"] == 21
+    own = [(int(x, 16), int(y, 16)) for x, y in run["contract_vk_points"]]
+    assert own[1] == vk_points[1] and own[0] != vk_points[0]      # only the range table coincides
+    cs = plonk_circuits.aggregation_shape()
+
+    def verdict(inst, prf, vk, t):
+        try:
+            return plonk_verifier.verify(cs, fx["k"], int(fx["vk_digest"]), vk[:4], vk[4:], [inst], prf, t)
+        except (AssertionError, ValueError):
+            return False
+    got = {name: verdict(*case) for name, case in yul_harness.cases(instances, proof, vk_points, own, tau).items()}
+    assert got == run["verdicts"]
+
+
+@pytest.mark.parametrize("path", _fixtures(), ids=lambda p: p.split("_")[-2])
+def test_independent_verifier_agrees_with_the_contract_term_by_term(orc, path):
     """VERDICT r1 item 8a: the independent Python verifier (tests/plonk_verifier.py) -- the check the multi-set / theta-lookup
     shapes rely on -- is pinned against the reference's verifier contract not only on accept / reject but on its intermediate
     values: every challenge it derives (theta, beta, gamma, y, x, and SHPLONK's y, v, u), x^n, the Lagrange terms l_0 and l_last,
-    the instance evaluation, the quotient numerator and the expected h(x) are words the contract itself stores while verifying
+    the instance evaluation, the quotient numerator and the expected h(x) are words the contract itself stored while verifying
     the same proof."""
-    import json
-    from tests import plonk_verifier, yul_harness
-    with open(path) as f:
-        fx = json.load(f)
-    contract = fx.get("contract", "sync_step_verifier")
-    instances = [int(v, 16) for v in fx["instances"]]
-    proof = bytes.fromhex(fx["proof"])
-    vk_points = [(int(x, 16), int(y, 16)) for x, y in fx["vk_points"]]
+    from tests import plonk_verifier
+    fx, run, instances, proof, vk_points = _contract_run(path)
+    assert run["verdicts"]["fixture"]
+    written = {int(w, 16) for w in run["stored_words"]}
     tau = orc.fr_ints(orc.srs_tau().reshape(1, 4))[0]
-    ok, m = yul_harness.run_contract(contract, instances, proof, vk_points, tau, kats)
-    assert ok
     trace = {}
     cs = plonk_circuits.aggregation_shape()
     assert plonk_verifier.verify(cs, fx["k"], int(fx["vk_digest"]), vk_points[:4], vk_points[4:], [instances], proof, tau, trace=trace)
     for name in ("theta", "beta", "gamma", "y", "x", "shplonk_y", "shplonk_v", "shplonk_u", "x_n", "l_0", "l_last", "quotient_numerator", "expected_h"):
-        assert trace[name] in m.written, "the contract never stores the verifier's %s" % name
+        assert trace[name] in written, "the contract never stores the verifier's %s" % name
     for q, v in trace["instance_evals"].items():
-        assert v in m.written, "instance evaluation %r" % (q,)
+        assert v in written, "instance evaluation %r" % (q,)
     # control: a value the contract has no reason to hold is not there by accident
-    assert (trace["theta"] + 1) % plonk.R_MOD not in m.written
+    assert (trace["theta"] + 1) % plonk.R_MOD not in written
 
 
 def test_halo2lib_sync_step_shape_proof_verifies(orc):

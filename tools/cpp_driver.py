@@ -9,12 +9,13 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def build_main_against_the_real_library():
-    """g++ tests/cpp/prover_main.cpp -DSPB_PROVER_WITH_CUDART against libspectre_b200.so + cudart -> tests/cpp/prover_main_cuda"""
+def build_main_against_the_real_library(out_dir=None):
+    """g++ tests/cpp/prover_main.cpp -DSPB_PROVER_WITH_CUDART against libspectre_b200.so + cudart -> prover_main_cuda in
+    out_dir (default tests/cpp/)"""
     from spectre_b200 import build
     lib = build.build()
     libdir = os.path.dirname(lib)
-    exe = os.path.join(ROOT, "tests", "cpp", "prover_main_cuda")
+    exe = os.path.join(out_dir or os.path.join(ROOT, "tests", "cpp"), "prover_main_cuda")
     src = os.path.join(ROOT, "tests", "cpp", "prover_main.cpp")
     hdrs = [os.path.join(ROOT, "include", h) for h in ("spectre_b200.h", "spectre_b200_prover.hpp")]
     if os.path.exists(exe) and os.path.getmtime(exe) >= max(os.path.getmtime(p) for p in [src, lib] + hdrs):
